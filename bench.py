@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU restatement of the reference
+    python bench.py ... --dump-outputs DIR                     # also write the last timed step's outputs
 
 Workload ("step" = one pass of the hot path over one batch of synthetic input): the full
 unsupervised FlowNetC training step of BASELINE.json configs[2]/[3] -- bidirectional FlowNetC
@@ -22,6 +23,12 @@ One JSON line on rank 0:
           no CPU path for this graph, SURVEY.md R1) on a bounded sample, timed on the host cores
   clocks  nvidia-smi SM clock / throttle reasons sampled (every 100 ms) during the timed region
 Timing: CUDA events on the launching stream, barrier + synchronize on both sides, max over ranks.
+--steps K sets the steps of every timed region: the headline and e2e regions run exactly K, the
+per-kernel eager pass (graph mode) and the fp32 pass at most K.
+--dump-outputs DIR: after the headline region, rank 0 writes what its last step returned to the
+caller as DIR/<name>.npy (float32): ``loss`` and, at the same DUMP_SAMPLE seeded flat positions, the
+updated trained variables (``params``) and Adam moments (``adam_m``, ``adam_v``).  Inputs and
+initial weights are seeded, so two builds run with the same arguments can be compared output for output.
 L2: one step streams several GB of activations (>> 126 MB L2), so no explicit flush is needed.
 """
 import argparse
@@ -37,12 +44,14 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
 from unflow_b200 import synthetic as synth  # noqa: E402
 
 H, W, PER_GPU_BATCH = 384, 1280, 4
+DUMP_SAMPLE = 1 << 21        # per array: 3 x 8 MB for FlowNetC's 39.2 M trained floats
 METRIC = "frame-pairs/s at 384x1280 FlowNetC"
 
 
@@ -139,6 +148,19 @@ def make_batch(rank, pinned):
 # ---------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, trainer, loss):
+    """The outputs of the step that just ran (see the module docstring); host copies."""
+    n = trainer.num_params
+    g = torch.Generator().manual_seed(0)
+    idx = torch.randperm(n, generator=g)[:min(n, DUMP_SAMPLE)].sort().values.to(trainer.device)
+    arrays = {"loss": loss.detach().float().reshape(1)}
+    for name, flat in (("params", trainer.flat_param), ("adam_m", trainer.adam_m), ("adam_v", trainer.adam_v)):
+        arrays[name] = flat[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy().astype(np.float32))
+
+
 def run_ours(args):
     from unflow_b200 import _native
     from unflow_b200.e2eflow import ops
@@ -176,8 +198,11 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def resident_step():
-        return trainer.step(d_im1, d_im2)
+        last["loss"] = trainer.step(d_im1, d_im2)
+        return last["loss"]
 
     sampler = ClockSampler(local)
     if rank == 0:
@@ -208,7 +233,7 @@ def run_ours(args):
         resident_step()
     # eager pass: per-kernel CUDA-event timings for the roofline objects (and the value itself when
     # graphs are off)
-    eager_steps = args.steps if not args.graph else max(3, min(args.steps, 5))
+    eager_steps = args.steps if not args.graph else min(args.steps, 5)
     ms, launches, ktimes, clocks = timed(resident_step, eager_steps, hook=True)
     kbytes = dict(ops.kernel_timer.bytes)
     steps_timed = eager_steps
@@ -220,6 +245,8 @@ def run_ours(args):
         ms, _, _, clocks = timed(resident_step, args.steps)
         launches = trainer._graph_launches * args.steps
         steps_timed = args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, last["loss"])
 
     def e2e_step():   # host batch -> (static) device buffers, step, loss back to the host
         if args.graph:
@@ -249,10 +276,11 @@ def run_ours(args):
         saved_graph, trainer._graph = trainer._graph, None     # eager: the captured graph is the 3xTF32 step
         for _ in range(3):
             resident_step()
-        ms32, _, _, _ = timed(resident_step, max(3, args.steps // 2))
+        steps32 = max(1, args.steps // 2)
+        ms32, _, _, _ = timed(resident_step, steps32)
         trainer._graph = saved_graph
-        fp32_exact = {"ms_per_step": round(ms32 / max(3, args.steps // 2), 3),
-                      "value": round(PER_GPU_BATCH * world / (ms32 / max(3, args.steps // 2) * 1e-3), 3),
+        fp32_exact = {"ms_per_step": round(ms32 / steps32, 3),
+                      "value": round(PER_GPU_BATCH * world / (ms32 / steps32 * 1e-3), 3),
                       "unit": "frame-pairs/s", "conv_precision": "fp32 (cuDNN, no tensor cores)"}
         conv_ops.set_mode(args.conv)
 
@@ -475,6 +503,9 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy "
+                         "(this repo's CUDA path only)")
     ap.add_argument("--prefetch", type=int, default=0,
                     help="1: overlap the host->device copy of the next batch with the running step in the "
                          "e2e loop (Trainer.prefetch / step_prefetched; opt-in, not yet measured)")
@@ -493,6 +524,8 @@ def main():
                     help="1 (default, N=1 only): additionally time the exact-fp32 conv mode (no tensor "
                          "cores) for a few steps and report it as fp32_exact next to the 3xTF32 headline")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

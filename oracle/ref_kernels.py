@@ -8,7 +8,8 @@ The op-registration files (*_op.cc) need the whole TensorFlow op framework and a
 the letter of the task the reference is therefore "unbuildable", what IS built are its GPU kernels
 and their launchers, which is where the arithmetic lives.
 
-Used by tests/test_reference_kernels.py (every ``-m gpu`` run) and tools/bench_reference_kernels.py.
+Used by tests/golden/make_reference_kernels.py (which stores their outputs for
+tests/test_reference_kernels.py) and tools/bench_reference_kernels.py.
 
 All functions take / return float32 CUDA tensors in the reference's layouts (correlation NCHW, the
 warps and downsample NHWC) and synchronise before returning; the kernels run on the legacy default
@@ -26,12 +27,12 @@ _lib = None
 
 
 def build():
-    """(Re)build when the reference tree is present (the build container) and fail loudly if that
-    leaves no library; where the tree is absent (the GPU box) the prebuilt file must have travelled."""
+    """(Re)build when the reference tree is present and fail loudly if that leaves no library; where
+    the tree is absent, a library built on another machine must have been copied to LIB_PATH."""
     subprocess.check_call(["bash", os.path.join(HERE, "ref_ops", "build.sh")])
     if not available():
-        raise RuntimeError("%s is missing: the reference kernels are the GPU ground truth of the "
-                           "parity tests (oracle/ref_ops/build.sh needs /root/reference)" % LIB_PATH)
+        raise RuntimeError("%s is missing: oracle/ref_ops/build.sh builds it from the reference tree "
+                           "(UNFLOW_REFERENCE)" % LIB_PATH)
 
 
 def available():

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Run the reference's OWN Python source (unmodified, from /root/reference/src/e2eflow/core) under
 the TensorFlow-API stand-in of tests/golden/tf_shim.py and store inputs + outputs as golden vectors
-in tests/golden/reference_run.npz.
+in tests/golden/reference_run.npz (seeded input images as their SHA-256, the full-resolution output
+flows as a fixed sample: tests/golden_data.py).
 
     python tests/golden/make_reference_run.py          (needs /root/reference; run in the build container)
 
@@ -26,8 +27,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
+sys.path.insert(0, os.path.dirname(HERE))
 REF_SRC = os.environ.get("UNFLOW_REFERENCE_SRC", "/root/reference/src")
 
+import golden_data  # noqa: E402
 import tf_shim  # noqa: E402
 from oracle import flownet as oflownet  # noqa: E402
 from oracle import ops as oops  # noqa: E402
@@ -320,6 +323,7 @@ def main():
                         'external': scope['restore_external_nets'], 'net_names': scope['net_names']}
     out['restore_plans_json'] = np.array(json.dumps(plans))
 
+    out = golden_data.shrink_reference_run(out)
     path = os.path.join(HERE, 'reference_run.npz')
     np.savez_compressed(path, **out)
     print("wrote %s: %d arrays, %.1f KB" % (path, len(out), os.path.getsize(path) / 1024.0))

@@ -2,8 +2,6 @@
 (tests/golden/reference_run.npz, see tests/golden/make_reference_run.py).  The tight comparisons
 are product-vs-oracle (other test files) and oracle-vs-vectors (CPU); this file closes the triangle
 directly, with tolerances one notch looser than those."""
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -11,9 +9,10 @@ import torch
 pytestmark = pytest.mark.gpu
 
 from oracle import flownet as oflownet
+import golden_data
 import synth
 
-G = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_run.npz"))
+G = golden_data.load_reference_run()
 WEIGHTS = dict(ternary=1.0, smooth_2nd=3.0, fb=0.2, occ=12.4, photo=0.5, grad=0.25, smooth_1st=0.75, sym=0.3)
 
 
@@ -79,5 +78,5 @@ def test_unsupervised_loss_against_reference_run(tag, spec, seed, extra):
         loss, ffw, fbw = unsupervised_loss((t('ul_%s_im1' % tag), t('ul_%s_im2' % tag)), params,
                                            synth.KITTI_NORMALIZATION, augment=False, return_flow=True, variables=v)
     close(loss, G['ul_%s_loss' % tag], rtol=1e-3, atol_rel=0.0)
-    close(ffw, G['ul_%s_flow_fw' % tag], rtol=1e-3, atol_rel=5e-4)
-    close(fbw, G['ul_%s_flow_bw' % tag], rtol=1e-3, atol_rel=5e-4)
+    close(*golden_data.run_flow(G, ffw, 'ul_%s_flow_fw' % tag), rtol=1e-3, atol_rel=5e-4)
+    close(*golden_data.run_flow(G, fbw, 'ul_%s_flow_bw' % tag), rtol=1e-3, atol_rel=5e-4)

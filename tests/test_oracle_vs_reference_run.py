@@ -12,9 +12,10 @@ from oracle import flownet as oflownet
 from oracle import image_warp as oimage_warp
 from oracle import losses as olosses
 from oracle import unsupervised as ounsup
+import golden_data
 import synth
 
-G = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_run.npz"))
+G = golden_data.load_reference_run()
 WEIGHTS = dict(ternary=1.0, smooth_2nd=3.0, fb=0.2, occ=12.4, photo=0.5, grad=0.25, smooth_1st=0.75, sym=0.3)
 
 
@@ -114,8 +115,8 @@ def test_unsupervised_loss_value_flows_and_gradients(tag, spec, seed, extra):
     loss, ffw, fbw = ounsup.unsupervised_loss(leaves, (t('ul_%s_im1' % tag), t('ul_%s_im2' % tag)), params,
                                               synth.KITTI_NORMALIZATION, augment=False, return_flow=True)
     close(loss, G['ul_%s_loss' % tag], rtol=2e-5)
-    close(ffw, G['ul_%s_flow_fw' % tag], rtol=1e-4, atol_rel=1e-5)
-    close(fbw, G['ul_%s_flow_bw' % tag], rtol=1e-4, atol_rel=1e-5)
+    close(*golden_data.run_flow(G, ffw, 'ul_%s_flow_fw' % tag), rtol=1e-4, atol_rel=1e-5)
+    close(*golden_data.run_flow(G, fbw, 'ul_%s_flow_bw' % tag), rtol=1e-4, atol_rel=1e-5)
     names = [str(n) for n in G['ul_%s_grad_names' % tag]]
     assert names == sorted(leaves)
     grads = torch.autograd.grad(loss, [leaves[k] for k in names], allow_unused=True)
@@ -126,7 +127,7 @@ def test_unsupervised_loss_value_flows_and_gradients(tag, spec, seed, extra):
     np.testing.assert_allclose(norms, want, rtol=2e-3)
     for k, g in zip(names, grads):
         key = 'ul_%s_grad/%s' % (tag, k)
-        if key in G.files:
+        if key in G:
             err = float((g - torch.from_numpy(G[key])).norm() / max(float(torch.from_numpy(G[key]).norm()), 1e-20))
             assert err < 2e-3, "%s: relative L2 gradient error %.2e" % (k, err)
 
@@ -320,8 +321,8 @@ def test_product_unsupervised_loss_host_path_on_the_cpu_against_the_reference_ru
     loss, ffw, fbw = U.unsupervised_loss((t('ul_%s_im1' % tag), t('ul_%s_im2' % tag)), params,
                                          synth.KITTI_NORMALIZATION, augment=False, return_flow=True, variables=v)
     close(loss, G['ul_%s_loss' % tag], rtol=2e-5)
-    close(ffw, G['ul_%s_flow_fw' % tag], rtol=1e-4, atol_rel=1e-5)
-    close(fbw, G['ul_%s_flow_bw' % tag], rtol=1e-4, atol_rel=1e-5)
+    close(*golden_data.run_flow(G, ffw, 'ul_%s_flow_fw' % tag), rtol=1e-4, atol_rel=1e-5)
+    close(*golden_data.run_flow(G, fbw, 'ul_%s_flow_bw' % tag), rtol=1e-4, atol_rel=1e-5)
     loss.backward()
     names = [str(n) for n in G['ul_%s_grad_names' % tag]]
     want = dict(zip(names, G['ul_%s_grad_norms' % tag]))
